@@ -9,6 +9,7 @@ weights / datasets exist offline, hence `data: synthetic`.
   python bench.py --gpus 1 --steps 5 --warmup 3            # our arm (CUDA kernels via the C ABI)
   python bench.py --impl reference --steps 2 --warmup 1     # the reference's CPU path (oracle port)
   torchrun ... bench.py --gpus N ...                        # one rank per GPU, weak scaling
+  python bench.py --steps 5 --warmup 3 --dump-outputs DIR   # also write the last timed step's outputs as DIR/<name>.npy
 
 Prints ONE JSON line (see README / DESIGN.md "Measurement").
 """
@@ -203,6 +204,36 @@ class Ctx:
     def close(self):
         if self.dist is not None:
             self.dist.destroy_process_group()
+
+
+DUMP_BUDGET_BYTES = 64 * 10 ** 6
+NPY_HEADER_BYTES = 256          # allowance per file for the .npy header (numpy writes 128 bytes for these shapes)
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BUDGET_BYTES, seed=0):
+    """Write each named tensor as <out_dir>/<name>.npy in float32 (the integer codes are < 2^24, exact in float32), at most
+    `budget` bytes in all, so that two builds run with the same arguments can be compared output for output.  The smallest
+    tensors are written whole; one that does not fit what is left is replaced by a seeded, sorted sample of its rows
+    (first dimension), with the sampled row indices beside it as <name>_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = budget
+    for name, t in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        a = t.detach().float().cpu()
+        rows_path = os.path.join(out_dir, f"{name}_rows.npy")
+        if os.path.exists(rows_path):           # from an earlier dump into the same directory
+            os.remove(rows_path)
+        if a.numel() * 4 + NPY_HEADER_BYTES > left:
+            n, row_bytes = a.shape[0], a[0].numel() * 4
+            k = (left - 2 * NPY_HEADER_BYTES) // (row_bytes + 8)
+            if k < 1:
+                raise ValueError(f"dump_outputs: no row of {name} {tuple(a.shape)} fits the {budget} byte budget")
+            rows = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:k].sort().values
+            a = a[rows]
+            np.save(rows_path, rows.double().numpy())
+            left -= rows.numel() * 8 + NPY_HEADER_BYTES
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+        left -= a.numel() * 4 + NPY_HEADER_BYTES
 
 
 def run_leg(ctx, sec, name, fn):
@@ -739,6 +770,7 @@ def run_codec(args, cfg, ctx, collect_secondary, first_legs=None):
             torch.cuda.synchronize()
     gbuf = {}
     tok_stack = torch.zeros(B, 2, 16, T // 3840, dtype=torch.int64, device=dev)
+    last = []                   # outputs of the latest step (the graph's static buffers: read before the next replay)
 
     def step_device():
         if graphed is not None:
@@ -750,7 +782,12 @@ def run_codec(args, cfg, ctx, collect_secondary, first_legs=None):
             tok_stack[:, 0].copy_(ac)
             tok_stack[:, 1].copy_(sc)
             gather_tokens(tok_stack, world * B, buffers=gbuf)
+        last[:] = (ac, sc, rec)
         return ac, sc, rec
+
+    def dump_last_step():
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dict(zip(("acoustic_codes", "semantic_codes", "wav_rec"), last)))
 
     codes_h = torch.empty(2, B, 16, T // 3840, dtype=torch.int64).pin_memory()
     rec_h = torch.empty(B, T).pin_memory()
@@ -785,6 +822,7 @@ def run_codec(args, cfg, ctx, collect_secondary, first_legs=None):
         for _ in range(args.warmup):
             step_device()
         ms = ctx.timed(step_device, args.steps)
+        dump_last_step()
         if rank == 0:
             print(json.dumps(dict(quick=True, ms_per_step=ms, value=world * B * T / (ms * 1e-3))))
         return None
@@ -797,6 +835,7 @@ def run_codec(args, cfg, ctx, collect_secondary, first_legs=None):
     ms = ctx.timed(step_device, args.steps)
     launches = ops.launch_count() + (graphed.launches_per_replay * args.steps if graphed is not None else 0)
     clocks = sampler.stop() if rank == 0 else None
+    dump_last_step()
     for _ in range(2):
         step_e2e()
     ms_e2e_serial = ctx.timed(step_e2e, args.steps)
@@ -1126,7 +1165,14 @@ def main():
                     help="all (default, the driver's line) = the codec line (BASELINE configs[1]) with the UniSE AR-LM legs (configs[2], [3], "
                          "[4]) under `secondary`; codec / lm / lm_tse / lm_forward / bicodec = that line alone")
     ap.add_argument("--quick", action="store_true", help="profiling aid: W warm-up + K steps only, no e2e/roofline/cpu legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed H-Codec-2.0 step returned (acoustic / semantic codes, "
+                         "waveform; rank 0) as DIR/<name>.npy in float32, at most 64 MB: a seeded sample of the waveform's clips if larger")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("all", "codec")):
+        ap.error("--dump-outputs writes the outputs of the H-Codec-2.0 step: --impl ours with --workload all or codec")
     args.warmup = max(args.warmup, 0)
     cfg = H2_FULL
     if args.workload == "bicodec":
